@@ -39,6 +39,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (it may be read-only)
 GiB, MiB = 1 << 30, 1 << 20
 BLOCK = 4 << 20
 METRIC = "GiB/s data-disk migration on Patch"
@@ -318,6 +319,48 @@ def parity_gate(vm, orc, src: Path, dst: Path, table: Path | None, ref_tree: Pat
             "gate_s": round(time.perf_counter() - t0, 1)}
 
 
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_STATS = ("bytes_total", "bytes_h2d", "bytes_d2h", "bytes_written", "blocks_total", "blocks_skipped", "files", "dirs",
+              "symlinks", "hardlinks", "specials", "pruned", "files_untrusted")
+DUMP_SAMPLE_BYTES = 1 << 20
+
+
+def dump_outputs(out_dir: Path, vm, dsts: list, tables: list, stats: dict) -> None:
+    """What the last timed step handed its caller, as .npy arrays, so that two builds can be compared output for output on
+    the same seeded workload: the block tables' XXH64 hashes (split into their 32-bit halves, which float64 holds exactly),
+    the statistics counters that do not depend on timing (in DUMP_STATS order), the size of every destination file and a
+    fixed, seeded sample of DUMP_SAMPLE_BYTES destination bytes.  Regular files are taken tree by tree, in bytewise path
+    order.  A few MB in all: 16 B per block, 8 B per file, 4 MB of sample."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    if tables:
+        h = np.concatenate([vm.table_hashes(t) for t in tables])
+        np.save(out_dir / "block_hash_hi32.npy", (h >> np.uint64(32)).astype(np.float64))
+        np.save(out_dir / "block_hash_lo32.npy", (h & np.uint64(0xFFFFFFFF)).astype(np.float64))
+    np.save(out_dir / "stats.npy", np.array([stats[k] for k in DUMP_STATS], dtype=np.float64))
+    files = []
+    for d in dsts:
+        tree = []
+        for dp, _dn, fn in os.walk(d):
+            for n in fn:
+                p = os.path.join(dp, n)
+                if os.path.isfile(p) and not os.path.islink(p):
+                    tree.append((os.fsencode(os.path.relpath(p, d)), p))
+        files += sorted(tree)
+    sizes = np.array([os.path.getsize(p) for _rel, p in files], dtype=np.int64)
+    np.save(out_dir / "dst_file_bytes.npy", sizes.astype(np.float64))
+    ends = np.cumsum(sizes)
+    total = int(ends[-1]) if len(ends) else 0
+    pos = np.sort(np.random.default_rng(20).integers(0, total, min(total, DUMP_SAMPLE_BYTES))) if total else np.empty(0, np.int64)
+    sample, lo = np.empty(len(pos), np.float32), 0
+    for (_rel, p), size, end in zip(files, sizes, ends):
+        hi = int(np.searchsorted(pos, end))
+        if hi > lo:
+            sample[lo:hi] = np.memmap(p, dtype=np.uint8, mode="r")[pos[lo:hi] - (end - size)]
+        lo = hi
+    np.save(out_dir / "dst_byte_sample.npy", sample)
+
+
 # ------------------------------------------------------------------------------------------------ reference arm
 def run_reference(args) -> None:
     """--impl reference: the reference's CPU implementation of the path on this box's host cores.  Its engine is
@@ -470,7 +513,13 @@ def main() -> None:
     ap.add_argument("--ref-sample-gib", type=int, default=20, help="reference arm, configs 3/4: GiB copied per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true", help="N>1, config 2A: skip rank 0's one-call-over-all-GPUs leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the engine's outputs; it does not apply to --impl reference")
     if args.warmup < 3:
         args.warmup = 3
     claim_stdout()
@@ -515,6 +564,7 @@ def main() -> None:
         d2h_bytes = 0
         n_gpu_used = 1 if not solo else n_gpus_box
         ref_tree = None
+        out_dsts, out_tables = [], []           # where the step leaves what it computed (--dump-outputs)
         clocks = ClockSampler(gpu)
 
         # ---------------- build the workload and the step
@@ -531,6 +581,7 @@ def main() -> None:
                 nbytes = datagen("files", src, plan["seed"], 10 * inproc_n, GiB) if cfg == "2A" else datagen("layer", src, 2, 10 * GiB, 40960)
                 mask = (all_mask if inproc_n > 1 else 1 << gpu) if cfg == "2A" else 1
                 n_gpu_used = inproc_n
+                out_dsts, out_tables = [base / "dst"], [base / "table.vmig"]
 
                 def step(i):
                     dst = fresh_dir(base / "dst")
@@ -545,6 +596,7 @@ def main() -> None:
             if active:
                 src = base / "src"
                 nbytes = datagen("files", src, 3, 100, GiB)
+                out_dsts, out_tables = [base / "dst"], [base / "table.vmig"]
 
                 def step(i):
                     dst = fresh_dir(base / "dst")
@@ -566,6 +618,7 @@ def main() -> None:
                 vm.hash_tree(dst, base / "v1.vmig", gpu_mask=all_mask)               # prior table = table of the pre-seeded dst
                 v1_want = oracle_table(orc, dst)
                 assert (vm.table_hashes(base / "v1.vmig") == v1_want).all(), "cfg4: prior table != oracle table of v1"
+                out_dsts, out_tables = [dst], [base / "v2.vmig"]
 
                 def step(i):
                     if i > 0:                       # outside the timed region: put dst back to v1 and re-take v1's table
@@ -592,6 +645,7 @@ def main() -> None:
                     nbytes += datagen("files", base / f"src{i}", 50 + i, 10, GiB)
                     srcs.append(base / f"src{i}")
                 per_call = [[] for _ in range(callers)]
+                out_dsts, out_tables = [base / f"dst{j}" for j in range(callers)], [base / f"t{j}.vmig" for j in range(callers)]
 
                 def step(i):
                     dsts = [fresh_dir(base / f"dst{j}") for j in range(callers)]
@@ -631,6 +685,7 @@ def main() -> None:
                 src = mnt.a / "src"
                 nbytes = GiB
                 want1 = None
+                out_dsts = [mnt.b / "dst"]
 
                 def step(i):
                     datagen("files", src, 1, 1, GiB)                 # the previous move emptied it
@@ -677,6 +732,8 @@ def main() -> None:
         elif not solo:
             pass
         clk = clocks.stop() if active else None
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, vm, out_dsts, out_tables, stats)
         if ref_tree is not None:
             shutil.rmtree(ref_tree, ignore_errors=True)
 

@@ -245,7 +245,7 @@ MetaPolicy default_meta_policy(uint32_t flags)
 
 static inline mode_t eff_mode(const Entry& e, const MetaPolicy& pol) {
     mode_t m = e.mode & 07777;
-    if (!pol.is_root) m &= ~pol.umask_bits & ~(mode_t)(S_ISUID | S_ISGID);   // tar without -p
+    if (!pol.is_root) m &= ~pol.umask_bits & 0777;   // tar without -p: umask applied, setuid/setgid/sticky dropped
     return m;
 }
 static inline void fill_times(const Entry& e, const MetaPolicy& pol, struct timespec ts[2]) {

@@ -95,6 +95,41 @@ def test_oracle_side_of_the_parity_gate(tmp_path):
         bench.parity_gate(FakeVm(), orc, src, dst, tmp_path / "t", None, "unit")
 
 
+def test_dump_outputs_writes_exact_float_arrays(tmp_path):
+    """--dump-outputs with a stand-in for the engine's table reader: the hashes come back exactly from their 32-bit halves,
+    file sizes and the seeded byte sample match the trees, and a second dump of the same trees is identical."""
+    src = tmp_path / "s"
+    (src / "x").mkdir(parents=True)
+    data = {"b.bin": os.urandom(3 * MiB + 5), "a.bin": b"", "x/c.bin": os.urandom(1000)}
+    for name, b in data.items():
+        (src / name).write_bytes(b)
+    os.symlink("b.bin", src / "lnk")
+    other = tmp_path / "o"
+    other.mkdir()
+    (other / "d.bin").write_bytes(os.urandom(MiB))
+
+    class FakeVm:
+        def table_hashes(self, path):
+            return {"t1": np.array([0, 1 << 63, (1 << 64) - 1], np.uint64), "t2": np.array([0x123456789ABCDEF0], np.uint64)}[path]
+    stats = {k: i for i, k in enumerate(bench.DUMP_STATS)}
+    stats["ns_total"] = 123
+    for d in ("d1", "d2"):
+        bench.dump_outputs(tmp_path / d, FakeVm(), [src, other], ["t1", "t2"], stats)
+    got = {p.stem: np.load(p) for p in (tmp_path / "d1").glob("*.npy")}
+    assert set(got) == {"block_hash_hi32", "block_hash_lo32", "stats", "dst_file_bytes", "dst_byte_sample"}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    h = (got["block_hash_hi32"].astype(np.uint64) << np.uint64(32)) | got["block_hash_lo32"].astype(np.uint64)
+    assert h.tolist() == [0, 1 << 63, (1 << 64) - 1, 0x123456789ABCDEF0]
+    assert got["stats"].tolist() == list(range(len(bench.DUMP_STATS)))
+    order = [data["a.bin"], data["b.bin"], data["x/c.bin"], (other / "d.bin").read_bytes()]
+    assert got["dst_file_bytes"].tolist() == [len(b) for b in order]
+    stream = np.frombuffer(b"".join(order), np.uint8)
+    pos = np.sort(np.random.default_rng(20).integers(0, stream.size, bench.DUMP_SAMPLE_BYTES))
+    assert (got["dst_byte_sample"] == stream[pos]).all()
+    for p in (tmp_path / "d2").glob("*.npy"):
+        assert (np.load(p) == got[p.stem]).all()
+
+
 def test_reference_arm_prints_exactly_one_json_line_on_stdout():
     """The contract is one JSON line on stdout; helpers and libraries may only write to stderr (config 1: the 1 GiB move)."""
     r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--config", "1", "--steps", "1", "--warmup", "3"],

@@ -76,13 +76,13 @@ def test_c_abi_from_plain_c(vm, shm_tmp):
         assert "no CPU fallback" in r.stdout and os.listdir(dst) == []
 
 
-def test_source_side_path_safety_unit(shm_tmp):
+def test_source_side_path_safety_unit(shm_tmp, tmp_path):
     """csrc/vmig_tree.cpp alone (no GPU, no CUDA): open_beneath refuses symlinks and escapes, the walk does not
     descend through symlinked directories, remove_source cannot be steered out of the tree; prune_extras (VMIG_F_PRUNE)
     removes exactly the entries the manifest lacks and never follows a symlink; the walk gives the same manifest with
-    one thread and with eight (hard-link pair across two sub-walks included)."""
+    one thread and with eight (hard-link pair across two sub-walks included); without root, modes follow tar without -p."""
     import subprocess
-    exe = shm_tmp / "tree_unit"
+    exe = tmp_path / "tree_unit"          # not /dev/shm: it may be mounted noexec
     csrc = ROOT / "gpu-docker-api_b200" / "csrc"
     subprocess.run(["g++", "-std=c++17", "-Wall", "-Werror", "-pthread", "-I", str(csrc), str(ROOT / "tests" / "tree_unit.cpp"),
                     str(csrc / "vmig_tree.cpp"), "-o", str(exe)], check=True)

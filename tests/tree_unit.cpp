@@ -117,6 +117,21 @@ int main(int argc, char** argv) {
         int links = 0; for (auto& e : b.files) if (e.hardlink_of >= 0) { links++; CHECK(b.files[(size_t)e.hardlink_of].rel == "d3/f0" && e.rel == "d9/hard"); }
         CHECK(links == 1);
     }
+
+    // ---- metadata as an ordinary user, like tar without -p: the umask applies, setuid/setgid/sticky bits are dropped
+    {
+        const std::string d = base + "/modes", f = d + "/suid";
+        CHECK(mkdir(d.c_str(), 0700) == 0);
+        put(f, "x");
+        const MetaPolicy pol{false, 022, false, false, false};
+        Entry e;
+        e.mtime = {1577934245, 0}; e.atime = {0, 0};
+        struct stat st;
+        e.rel = "modes/suid"; e.type = kFile; e.mode = S_IFREG | 04770;
+        CHECK(apply_file_meta(-1, f, e, pol) == VMIG_OK && stat(f.c_str(), &st) == 0 && (st.st_mode & 07777) == 0750);
+        e.rel = "modes"; e.type = kDir; e.mode = S_IFDIR | 03777;
+        CHECK(apply_file_meta(-1, d, e, pol) == VMIG_OK && stat(d.c_str(), &st) == 0 && (st.st_mode & 07777) == 0755);
+    }
     printf("tree unit ok\n");
     return 0;
 }
