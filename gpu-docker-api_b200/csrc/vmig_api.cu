@@ -23,6 +23,29 @@ namespace {
 
 inline std::string pjoin(const std::string& a, const std::string& b) { return b == "." ? a : a + "/" + b; }
 
+inline int64_t ctime_ns(const struct stat& st) { return (int64_t)st.st_ctim.tv_sec * 1000000000ll + st.st_ctim.tv_nsec; }
+
+// Opens destination file p for writing, O_DIRECT if *direct; *direct then says whether O_DIRECT took.  create: a new
+// file, replacing what is there like tar does (a directory in the way is an error); else the existing file.  A
+// filesystem that refuses O_DIRECT (EINVAL) gets the same open without it, and without O_EXCL: the refused attempt may
+// already have created the file.
+int open_for_write(const std::string& p, bool create, bool* direct, int* out)
+{
+    if (create) {
+        bool was_dir = false;
+        int rc = unlink_if_exists(p, &was_dir);
+        if (rc) return rc;
+        if (was_dir) return fail(VMIG_EIO, "%s: a directory is in the way of a regular file", p.c_str());
+    }
+    const int flags = O_WRONLY | O_CLOEXEC | O_NOFOLLOW | (create ? O_CREAT | O_EXCL : 0);
+    const bool want = *direct;
+    *out = open(p.c_str(), flags | (want ? O_DIRECT : 0), 0600);
+    *direct = want && *out >= 0;
+    if (*out < 0 && want && errno == EINVAL) *out = open(p.c_str(), flags & ~O_EXCL, 0600);
+    if (*out < 0) return fail(VMIG_EIO, "open %s for writing: %s", p.c_str(), errno_str(errno).c_str());
+    return VMIG_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 // file-backed BlockIO
 class FileIO : public BlockIO {
@@ -36,6 +59,7 @@ public:
         bool s_direct = false, d_direct = false;         // this file's descriptor was opened with O_DIRECT
         std::atomic<void*> s_cfh{nullptr}, d_cfh{nullptr};   // cuFile handles of sfd / dfd (VMIG_F_CUFILE)
         std::atomic<bool> wrote{false};                  // at least one block of the file was written in this call
+        void set_identity(const struct stat& st) { id_ino = (uint64_t)st.st_ino; id_ctime_ns = ctime_ns(st); }
     };
     std::string src_root, dst_root;
     int src_root_fd = -1;                // source files are opened beneath this descriptor, never by absolute path
@@ -53,12 +77,37 @@ public:
     std::unique_ptr<FS[]> fs;
     std::mutex stripes[64];
 
+    // One pass over man's files, reading them beneath `root`: every file with blocks of its own is opened at its first
+    // block and closed after its last.
+    int setup(const std::string& root, const Manifest& man) {
+        src_root = root; m = &man;
+        fs.reset(new FS[man.files.size() ? man.files.size() : 1]);
+        for (size_t f = 0; f < man.files.size(); f++) {
+            const Entry& e = man.files[f];
+            if (e.hardlink_of >= 0 || e.n_blocks == 0) continue;
+            fs[f].reads_left.store((uint32_t)e.n_blocks); fs[f].blocks_left.store((uint32_t)e.n_blocks);
+        }
+        if (cufile) { int rc = cufile_open(); if (rc) return rc; }
+        src_root_fd = open(src_root.c_str(), O_RDONLY | O_DIRECTORY | O_CLOEXEC);
+        if (src_root_fd < 0) return fail(VMIG_EIO, "open %s: %s", src_root.c_str(), errno_str(errno).c_str());
+        return VMIG_OK;
+    }
+    ~FileIO() { close_all(); if (src_root_fd >= 0) close(src_root_fd); }
+
+    // Swaps *fd for a descriptor registered with libcufile, whose handle goes to h; *fd is closed on failure.
     // libcufile refuses descriptors whose open flags include O_NOFOLLOW / O_NONBLOCK ("unsupported file open flags"),
     // which is exactly how the safe opens below are made, and F_SETFL cannot clear O_NOFOLLOW.  The descriptor already
     // refers to the checked regular file, so it is re-opened through /proc/self/fd with plain flags.
-    static int reopen_plain(int fd, int flags) {
-        char p[64]; snprintf(p, sizeof p, "/proc/self/fd/%d", fd);
-        return open(p, flags | O_CLOEXEC);
+    static int cufile_attach(int* fd, int flags, const std::string& name, std::atomic<void*>& h) {
+        char path[64]; snprintf(path, sizeof path, "/proc/self/fd/%d", *fd);
+        const int nfd = open(path, flags | O_CLOEXEC);
+        if (nfd < 0) { const int e = errno; close(*fd); return fail(VMIG_EIO, "reopen %s for cuFile: %s", name.c_str(), errno_str(e).c_str()); }
+        close(*fd); *fd = nfd;
+        void* handle = nullptr;
+        const int rc = cufile_handle_open(nfd, &handle);
+        if (rc) { close(nfd); return rc; }
+        h.store(handle, std::memory_order_release);
+        return VMIG_OK;
     }
     int open_src(uint32_t f, int* out) {
         FS& s = fs[f];
@@ -78,17 +127,9 @@ public:
                     close(fd);
                     return fail(VMIG_ESRCCHANGED, "%s is not a regular file any more", m->files[f].rel.c_str());
                 }
-                if (hash_only && st.st_nlink == 1) { s.id_ino = (uint64_t)st.st_ino; s.id_ctime_ns = (int64_t)st.st_ctim.tv_sec * 1000000000ll + st.st_ctim.tv_nsec; }
+                if (hash_only && st.st_nlink == 1) s.set_identity(st);
                 if (s.s_direct) n_direct++;
-                if (cufile) {
-                    const int nfd = reopen_plain(fd, O_RDONLY | (s.s_direct ? O_DIRECT : 0));
-                    if (nfd < 0) { const int e = errno; close(fd); return fail(VMIG_EIO, "reopen %s for cuFile: %s", m->files[f].rel.c_str(), errno_str(e).c_str()); }
-                    close(fd); fd = nfd;
-                    void* h = nullptr;
-                    rc = cufile_handle_open(fd, &h);
-                    if (rc) { close(fd); return rc; }
-                    s.s_cfh.store(h, std::memory_order_release);
-                }
+                if (cufile) { rc = cufile_attach(&fd, O_RDONLY | (s.s_direct ? O_DIRECT : 0), m->files[f].rel, s.s_cfh); if (rc) return rc; }
                 s.sfd.store(fd, std::memory_order_release);
             }
         }
@@ -102,51 +143,31 @@ public:
             fd = s.dfd.load(std::memory_order_acquire);
             if (fd < 0) {
                 const std::string p = pjoin(dst_root, m->files[f].rel);
-                const int dflag = direct && corrupt_block < 0 ? O_DIRECT : 0;
-                if (s.inplace) {
-                    fd = open(p.c_str(), O_WRONLY | O_CLOEXEC | O_NOFOLLOW | dflag);
-                    if (fd < 0 && dflag && errno == EINVAL) fd = open(p.c_str(), O_WRONLY | O_CLOEXEC | O_NOFOLLOW); else s.d_direct = dflag != 0 && fd >= 0;
-                } else {
-                    bool was_dir = false;
-                    int rc = unlink_if_exists(p, &was_dir);     // tar replaces what is there
-                    if (rc) return rc;
-                    if (was_dir) return fail(VMIG_EIO, "%s: a directory is in the way of a regular file", p.c_str());
-                    fd = open(p.c_str(), O_WRONLY | O_CREAT | O_EXCL | O_CLOEXEC | O_NOFOLLOW | dflag, 0600);
-                    if (fd < 0 && dflag && errno == EINVAL) fd = open(p.c_str(), O_WRONLY | O_CREAT | O_CLOEXEC | O_NOFOLLOW, 0600); else s.d_direct = dflag != 0 && fd >= 0;
-                }
-                if (fd < 0) return fail(VMIG_EIO, "open %s for writing: %s", p.c_str(), errno_str(errno).c_str());
-                if (s.d_direct) n_direct++;
-                if (cufile && !hash_only) {
-                    const int nfd = reopen_plain(fd, O_WRONLY | (s.d_direct ? O_DIRECT : 0));
-                    if (nfd < 0) { const int e = errno; close(fd); return fail(VMIG_EIO, "reopen %s for cuFile: %s", p.c_str(), errno_str(e).c_str()); }
-                    close(fd); fd = nfd;
-                    void* h = nullptr;
-                    int rc = cufile_handle_open(fd, &h);
-                    if (rc) { close(fd); return rc; }
-                    s.d_cfh.store(h, std::memory_order_release);
-                }
+                bool dio = direct && corrupt_block < 0;       // the fault hook's one-byte pwrite cannot be O_DIRECT
+                int rc = open_for_write(p, !s.inplace, &dio, &fd);
+                if (rc) return rc;
+                s.d_direct = dio;
+                if (dio) n_direct++;
+                if (cufile && !hash_only) { rc = cufile_attach(&fd, O_WRONLY | (dio ? O_DIRECT : 0), p, s.d_cfh); if (rc) return rc; }
                 s.dfd.store(fd, std::memory_order_release);
             }
         }
         *out = fd; return VMIG_OK;
     }
+    // O_DIRECT: buffer, offset and length in whole sectors (the slot layout leaves the room; the device DMAs straight
+    // into the pinned ring)
     int read_block(const BlockRef& b, uint8_t* dst) override {
         int fd; int rc = open_src(b.file, &fd);
         if (rc) return rc;
         FS& s = fs[b.file];
-        // O_DIRECT: buffer, offset and length in whole sectors (the slot layout leaves the room; the device DMAs straight
-        // into the pinned ring); the file's last block is short, the read past EOF simply returns fewer bytes
-        const size_t want = s.s_direct ? (size_t)align_up(b.len, kSector) : b.len;
-        size_t got = 0;
-        while (got < b.len) {
-            const size_t pos = s.s_direct ? (got & ~(size_t)(kSector - 1)) : got;      // after a short direct read: back to a sector boundary
-            ssize_t r = pread(fd, dst + pos, want - pos, (off_t)(b.file_off + pos));
-            if (r < 0) { if (errno == EINTR) continue; return fail(VMIG_EIO, "pread %s: %s", m->files[b.file].rel.c_str(), errno_str(errno).c_str()); }
-            if (r == 0 || pos + (size_t)r <= got) return fail(VMIG_ESRCCHANGED, "%s shrank while being migrated (wanted %u bytes at %llu, got %zu)", m->files[b.file].rel.c_str(), b.len, (unsigned long long)b.file_off, got);
-            got = pos + (size_t)r;
-        }
-        if (s.reads_left.fetch_sub(1) == 1) { close_src(s, fd); }
-        return VMIG_OK;
+        const char* name = m->files[b.file].rel.c_str();
+        rc = transfer_block(name, b.file_off, b.len, s.s_direct ? kSector : 0, VMIG_ESRCCHANGED, [&](size_t pos, size_t n) -> ssize_t {
+            ssize_t r;
+            while ((r = pread(fd, dst + pos, n, (off_t)(b.file_off + pos))) < 0 && errno == EINTR) {}
+            return r < 0 ? fail(VMIG_EIO, "pread %s: %s", name, errno_str(errno).c_str()) : r;
+        });
+        if (!rc && s.reads_left.fetch_sub(1) == 1) close_src(s, fd);
+        return rc;
     }
     void close_src(FS& s, int fd) {
         void* h = s.s_cfh.exchange(nullptr);
@@ -159,17 +180,11 @@ public:
         if (rc) return rc;
         FS& s = fs[b.file];
         void* h = s.s_cfh.load(std::memory_order_acquire);
-        const size_t want = s.s_direct ? (size_t)align_up(b.len, kSector) : b.len;
-        size_t got = 0;
-        while (got < b.len) {
-            const size_t pos = s.s_direct ? (got & ~(size_t)(kSector - 1)) : got;
-            const ssize_t r = cufile_read(h, d_base, want - pos, (off_t)(b.file_off + pos), (off_t)(d_off + pos));
-            if (r < 0) return (int)r;
-            if (r == 0 || pos + (size_t)r <= got) return fail(VMIG_ESRCCHANGED, "%s shrank while being migrated (wanted %u bytes at %llu, got %zu)", m->files[b.file].rel.c_str(), b.len, (unsigned long long)b.file_off, got);
-            got = pos + (size_t)r;
-        }
-        if (s.reads_left.fetch_sub(1) == 1) close_src(s, fd);
-        return VMIG_OK;
+        rc = transfer_block(m->files[b.file].rel.c_str(), b.file_off, b.len, s.s_direct ? kSector : 0, VMIG_ESRCCHANGED, [&](size_t pos, size_t n) {
+            return cufile_read(h, d_base, n, (off_t)(b.file_off + pos), (off_t)(d_off + pos));
+        });
+        if (!rc && s.reads_left.fetch_sub(1) == 1) close_src(s, fd);
+        return rc;
     }
     // GPUDirect Storage: HBM slot -> file (surviving blocks only)
     int write_block_dev(const BlockRef& b, const uint8_t* d_base, size_t d_off) override {
@@ -178,42 +193,26 @@ public:
         FS& s = fs[b.file];
         s.wrote.store(true, std::memory_order_relaxed);
         void* h = s.d_cfh.load(std::memory_order_acquire);
-        const size_t want = s.d_direct ? (size_t)align_up(b.len, kSector) : b.len;
-        size_t put = 0;
-        while (put < b.len) {
-            const size_t pos = s.d_direct ? (put & ~(size_t)(kSector - 1)) : put;
-            const ssize_t w = cufile_write(h, d_base, want - pos, (off_t)(b.file_off + pos), (off_t)(d_off + pos));
-            if (w < 0) return (int)w;
-            if (w == 0 || pos + (size_t)w <= put) return fail(VMIG_EIO, "cuFileWrite %s: wrote 0 bytes", m->files[b.file].rel.c_str());
-            put = pos + (size_t)w;
-        }
-        return VMIG_OK;
+        return transfer_block(m->files[b.file].rel.c_str(), b.file_off, b.len, s.d_direct ? kSector : 0, VMIG_EIO, [&](size_t pos, size_t n) {
+            return cufile_write(h, d_base, n, (off_t)(b.file_off + pos), (off_t)(d_off + pos));
+        });
     }
+    // O_DIRECT: whole sectors out of the pinned ring; a short last block is written padded (whatever follows it in the
+    // slot) and block_done() cuts the file back to its size
     int write_block(const BlockRef& b, const uint8_t* src) override {
         int fd; int rc = open_dst(b.file, &fd);
         if (rc) return rc;
-        fs[b.file].wrote.store(true, std::memory_order_relaxed);
-        if (corrupt_block >= 0 && (uint64_t)corrupt_block == b.table_idx && b.len) {
-            const uint8_t bad = src[0] ^ 1u;           // what VMIG_F_VERIFY exists to catch
-            if (pwrite(fd, &bad, 1, (off_t)b.file_off) != 1) return fail(VMIG_EIO, "pwrite (fault hook)");
-            if (b.len == 1) return VMIG_OK;
-            size_t put1 = 1;
-            while (put1 < b.len) { ssize_t w = pwrite(fd, src + put1, b.len - put1, (off_t)(b.file_off + put1)); if (w <= 0) return fail(VMIG_EIO, "pwrite (fault hook)"); put1 += (size_t)w; }
-            return VMIG_OK;
-        }
-        // O_DIRECT: whole sectors out of the pinned ring; a short last block is written padded (whatever follows it in the
-        // slot) and block_done() cuts the file back to its size
-        const bool dio = fs[b.file].d_direct;
-        const size_t want = dio ? (size_t)align_up(b.len, kSector) : b.len;
-        size_t put = 0;
-        while (put < b.len) {
-            const size_t pos = dio ? (put & ~(size_t)(kSector - 1)) : put;
-            ssize_t w = pwrite(fd, src + pos, want - pos, (off_t)(b.file_off + pos));
-            if (w < 0) { if (errno == EINTR) continue; return fail(VMIG_EIO, "pwrite %s: %s", m->files[b.file].rel.c_str(), errno_str(errno).c_str()); }
-            if (w == 0 || pos + (size_t)w <= put) return fail(VMIG_EIO, "pwrite %s: wrote 0 bytes", m->files[b.file].rel.c_str());
-            put = pos + (size_t)w;
-        }
-        return VMIG_OK;
+        FS& s = fs[b.file];
+        s.wrote.store(true, std::memory_order_relaxed);
+        const char* name = m->files[b.file].rel.c_str();
+        rc = transfer_block(name, b.file_off, b.len, s.d_direct ? kSector : 0, VMIG_EIO, [&](size_t pos, size_t n) -> ssize_t {
+            ssize_t w;
+            while ((w = pwrite(fd, src + pos, n, (off_t)(b.file_off + pos))) < 0 && errno == EINTR) {}
+            return w < 0 ? fail(VMIG_EIO, "pwrite %s: %s", name, errno_str(errno).c_str()) : w;
+        });
+        if (rc || corrupt_block < 0 || (uint64_t)corrupt_block != b.table_idx || !b.len) return rc;
+        const uint8_t bad = src[0] ^ 1u;           // what VMIG_F_VERIFY exists to catch
+        return pwrite(fd, &bad, 1, (off_t)b.file_off) == 1 ? VMIG_OK : fail(VMIG_EIO, "pwrite (fault hook)");
     }
     int block_done(const BlockRef& b, bool) override {
         FS& s = fs[b.file];
@@ -231,20 +230,14 @@ public:
         const bool untouched = s.inplace && !s.wrote.load() && s.dst_old_size == e.size && file_meta_matches(fd, e, pol);
         rc = untouched ? VMIG_OK : apply_file_meta(fd, p, e, pol);
         struct stat ids;                             // nothing touches the file after this point: its ctime is final
-        if (!rc && fstat(fd, &ids) == 0) { s.id_ino = (uint64_t)ids.st_ino; s.id_ctime_ns = (int64_t)ids.st_ctim.tv_sec * 1000000000ll + ids.st_ctim.tv_nsec; }
+        if (!rc && fstat(fd, &ids) == 0) s.set_identity(ids);
         { void* h = s.d_cfh.exchange(nullptr); if (h) cufile_handle_close(h); }
         if (close(fd) != 0 && !rc) rc = fail(VMIG_EIO, "close %s: %s", p.c_str(), errno_str(errno).c_str());
         s.dfd.store(-1);
         return rc;
     }
-    int open_root() {
-        src_root_fd = open(src_root.c_str(), O_RDONLY | O_DIRECTORY | O_CLOEXEC);
-        if (src_root_fd < 0) return fail(VMIG_EIO, "open %s: %s", src_root.c_str(), errno_str(errno).c_str());
-        return VMIG_OK;
-    }
-    ~FileIO() { if (src_root_fd >= 0) close(src_root_fd); }
-    void close_all(size_t n) {
-        for (size_t i = 0; i < n; i++) {
+    void close_all() {
+        for (size_t i = 0; fs && i < m->files.size(); i++) {
             void* h = fs[i].s_cfh.exchange(nullptr); if (h) cufile_handle_close(h);
             h = fs[i].d_cfh.exchange(nullptr); if (h) cufile_handle_close(h);
             int a = fs[i].sfd.exchange(-1); if (a >= 0) close(a);
@@ -353,67 +346,45 @@ int run_blocks(const std::vector<BlockRef>& blocks, BlockIO* io, bool has_prior,
     return VMIG_OK;
 }
 
-vmig_opts norm_opts(const vmig_opts* in) {
-    vmig_opts o; memset(&o, 0, sizeof o);
-    if (in) o = *in;
-    if (!o.block_bytes) o.block_bytes = 4u << 20;
-    if (env_long("VMIG_DIRECT_IO", 0) == 1) o.flags |= VMIG_F_DIRECT_IO;
-    if (env_long("VMIG_CUFILE", 0) == 1) o.flags |= VMIG_F_CUFILE;
-    return o;
+int norm_opts(const vmig_opts* in, vmig_opts* o) {
+    memset(o, 0, sizeof *o);
+    if (in) *o = *in;
+    if (!o->block_bytes) o->block_bytes = 4u << 20;
+    if (env_long("VMIG_DIRECT_IO", 0) == 1) o->flags |= VMIG_F_DIRECT_IO;
+    if (env_long("VMIG_CUFILE", 0) == 1) o->flags |= VMIG_F_CUFILE;
+    if (o->block_bytes & 4095u) return fail(VMIG_EINVAL, "block_bytes %u is not a multiple of 4096", o->block_bytes);
+    if (o->block_bytes > pipe_slot_bytes()) return fail(VMIG_EINVAL, "block_bytes %u exceeds the staging slot (%u)", o->block_bytes, pipe_slot_bytes());
+    return VMIG_OK;
 }
 
-int migrate_tree_impl(const char* src_dir, const char* dst_dir, const char* prior_path, const char* out_path,
-                      const vmig_opts* opts_in, vmig_stats* stats_out)
+// The arguments, before anything is touched: both directories are there, and so is a GPU (no CPU fallback).
+int check_args(const char* src_dir, const char* dst_dir, const vmig_opts* opts_in, vmig_opts* o)
 {
-    vmig_stats st; memset(&st, 0, sizeof st);
-    const uint64_t t_begin = now_ns();
     if (!src_dir || !*src_dir) return fail(VMIG_EINVAL, "src_dir is NULL/empty");
-    vmig_opts o = norm_opts(opts_in);
-    const bool hash_only = (o.flags & VMIG_F_HASH_ONLY) != 0;
+    int rc = norm_opts(opts_in, o);
+    if (rc) return rc;
+    const bool hash_only = (o->flags & VMIG_F_HASH_ONLY) != 0;
     if (!hash_only && (!dst_dir || !*dst_dir)) return fail(VMIG_EINVAL, "dst_dir is NULL/empty");
-    if (o.block_bytes & 4095u) return fail(VMIG_EINVAL, "block_bytes %u is not a multiple of 4096", o.block_bytes);
-    if (o.block_bytes > pipe_slot_bytes()) return fail(VMIG_EINVAL, "block_bytes %u exceeds the staging slot (%u)", o.block_bytes, pipe_slot_bytes());
-    const std::string src(src_dir), dst(dst_dir ? dst_dir : "");
     struct stat sst;
-    if (stat(src.c_str(), &sst) != 0) return fail(VMIG_EIO, "stat %s: %s", src.c_str(), errno_str(errno).c_str());
-    if (!S_ISDIR(sst.st_mode)) return fail(VMIG_ENOTDIR, "%s is not a directory", src.c_str());
+    if (stat(src_dir, &sst) != 0) return fail(VMIG_EIO, "stat %s: %s", src_dir, errno_str(errno).c_str());
+    if (!S_ISDIR(sst.st_mode)) return fail(VMIG_ENOTDIR, "%s is not a directory", src_dir);
     if (!hash_only) {
-        if (stat(dst.c_str(), &sst) != 0) return fail(VMIG_EIO, "stat %s: %s", dst.c_str(), errno_str(errno).c_str());
-        if (!S_ISDIR(sst.st_mode)) return fail(VMIG_ENOTDIR, "%s is not a directory", dst.c_str());
+        if (stat(dst_dir, &sst) != 0) return fail(VMIG_EIO, "stat %s: %s", dst_dir, errno_str(errno).c_str());
+        if (!S_ISDIR(sst.st_mode)) return fail(VMIG_ENOTDIR, "%s is not a directory", dst_dir);
     }
-    // make sure a GPU is there before touching the destination: no CPU fallback
     std::vector<DeviceInfo> devs;
-    int rc = ctx_select(o.gpu_mask, &devs);
-    if (rc) return rc;
+    return ctx_select(o->gpu_mask, &devs);
+}
 
-    Manifest man;
-    uint64_t t0 = now_ns();
-    rc = walk_tree(src, o.block_bytes, (o.flags & VMIG_F_SKIP_HIDDEN_TOPDIRS) != 0, &man);
-    if (rc) return rc;
-    st.ns_walk = now_ns() - t0;
-
-    t0 = now_ns();
-    BlockTable prior; bool has_prior = false;
-    if (prior_path && *prior_path && !hash_only) {
-        rc = table_load(prior_path, &prior);
-        if (rc) return rc;
-        if (prior.block_bytes != o.block_bytes) return fail(VMIG_ETABLE, "prior table block size %u != %u", prior.block_bytes, o.block_bytes);
-        has_prior = true;
-    }
-    FileIO io;
-    io.src_root = src; io.dst_root = dst; io.m = &man; io.pol = default_meta_policy(o.flags); io.hash_only = hash_only;
-    io.corrupt_block = env_long("VMIG_CORRUPT_BLOCK", -1);
-    io.direct = (o.flags & VMIG_F_DIRECT_IO) != 0;
-    io.cufile = (o.flags & VMIG_F_CUFILE) != 0;
-    if (io.cufile) { rc = cufile_open(); if (rc) return rc; }
-    rc = io.open_root(); if (rc) return rc;
-    io.fs.reset(new FileIO::FS[man.files.size() ? man.files.size() : 1]);
-    std::vector<uint64_t> hashes(man.n_blocks, 0);
-
-    // ---- per-file state + block list.  Files are taken in groups of 64 (bounds open fds) and
-    // blocks round-robin across the group's files so many destination files are written at once
-    // (a single tmpfs/xfs file takes writes one thread at a time: profiles/r01_hostio_probe.txt).
-    std::vector<BlockRef> blocks; blocks.reserve(man.n_blocks);
+// Per-file state and the block list.  A destination file that still IS the one the prior table was written for (same
+// inode, same ctime -- any write, truncate, chmod or replacement since then moved it --, same size) is patched in place;
+// one the table names but that changed since is counted in *untrusted and rewritten.  Files are taken in groups of 64
+// (bounds open fds) and blocks round-robin across the group's files so many destination files are written at once (a
+// single tmpfs/xfs file takes writes one thread at a time: profiles/r01_hostio_probe.txt).
+void plan_blocks(const Manifest& man, const BlockTable* prior, uint32_t block_bytes, FileIO& io,
+                 std::vector<BlockRef>* blocks, uint64_t* untrusted)
+{
+    blocks->reserve(man.n_blocks);
     std::vector<uint32_t> group;
     auto flush_group = [&]() {
         uint64_t maxb = 0;
@@ -422,35 +393,30 @@ int migrate_tree_impl(const char* src_dir, const char* dst_dir, const char* prio
             for (uint32_t f : group) {
                 const Entry& e = man.files[f];
                 if (r >= e.n_blocks) continue;
-                BlockRef b; b.file = f; b.file_off = r * (uint64_t)o.block_bytes;
-                b.len = (uint32_t)std::min<uint64_t>(o.block_bytes, e.size - b.file_off);
+                BlockRef b; b.file = f; b.file_off = r * (uint64_t)block_bytes;
+                b.len = (uint32_t)std::min<uint64_t>(block_bytes, e.size - b.file_off);
                 b.table_idx = e.first_block + r; b.prior_hash = 0; b.prior_valid = 0;
                 if (io.fs[f].inplace) {
-                    const TableFile& pf = prior.files[prior.index[e.rel]];
-                    const uint64_t plen = r < prior.blocks_of(pf) ? std::min<uint64_t>(o.block_bytes, pf.size - b.file_off) : 0;
-                    if (plen == b.len) { b.prior_hash = prior.hashes[pf.first_block + r]; b.prior_valid = 1; }
+                    const TableFile& pf = prior->files[prior->index.at(e.rel)];
+                    const uint64_t plen = r < prior->blocks_of(pf) ? std::min<uint64_t>(block_bytes, pf.size - b.file_off) : 0;
+                    if (plen == b.len) { b.prior_hash = prior->hashes[pf.first_block + r]; b.prior_valid = 1; }
                 }
-                blocks.push_back(b);
+                blocks->push_back(b);
             }
         group.clear();
     };
     for (uint32_t f = 0; f < man.files.size(); f++) {
         const Entry& e = man.files[f];
         if (e.hardlink_of >= 0 || e.n_blocks == 0) continue;
-        FileIO::FS& s = io.fs[f];
-        s.reads_left.store((uint32_t)e.n_blocks); s.blocks_left.store((uint32_t)e.n_blocks);
-        if (has_prior) {
-            auto it = prior.index.find(e.rel);
+        if (prior) {
+            auto it = prior->index.find(e.rel);
             struct stat ds;
-            // patch in place only a destination file that still IS the one the table was written for: same
-            // inode, same ctime (any write, truncate, chmod or replacement since then moved it), same size
-            if (it != prior.index.end() && lstat(pjoin(dst, e.rel).c_str(), &ds) == 0 && S_ISREG(ds.st_mode) && ds.st_nlink == 1) {
-                const TableFile& pf = prior.files[it->second];
-                const int64_t ct = (int64_t)ds.st_ctim.tv_sec * 1000000000ll + ds.st_ctim.tv_nsec;
-                if (pf.ino != 0 && (uint64_t)ds.st_ino == pf.ino && ct == pf.ctime_ns && (uint64_t)ds.st_size == pf.size) {
-                    s.inplace = true; s.dst_old_size = (uint64_t)ds.st_size;
+            if (it != prior->index.end() && lstat(pjoin(io.dst_root, e.rel).c_str(), &ds) == 0 && S_ISREG(ds.st_mode) && ds.st_nlink == 1) {
+                const TableFile& pf = prior->files[it->second];
+                if (pf.ino != 0 && (uint64_t)ds.st_ino == pf.ino && ctime_ns(ds) == pf.ctime_ns && (uint64_t)ds.st_size == pf.size) {
+                    io.fs[f].inplace = true; io.fs[f].dst_old_size = (uint64_t)ds.st_size;
                 } else if (pf.ino != 0) {
-                    st.files_untrusted++;
+                    (*untrusted)++;
                 }
             }
         }
@@ -458,6 +424,116 @@ int migrate_tree_impl(const char* src_dir, const char* dst_dir, const char* prio
         if (group.size() == 64) flush_group();
     }
     flush_group();
+}
+
+// empty regular files carry no blocks: created here, after the data pass
+int create_empty_files(const Manifest& man, FileIO& io)
+{
+    for (size_t f = 0; f < man.files.size(); f++) {
+        const Entry& e = man.files[f];
+        if (e.hardlink_of >= 0 || e.n_blocks) continue;
+        const std::string p = pjoin(io.dst_root, e.rel);
+        bool dio = false; int fd;
+        int rc = open_for_write(p, true, &dio, &fd);
+        if (rc) return rc;
+        rc = apply_file_meta(fd, p, e, io.pol);
+        struct stat ids;
+        if (!rc && fstat(fd, &ids) == 0) io.fs[f].set_identity(ids);
+        close(fd);
+        if (rc) return rc;
+    }
+    return VMIG_OK;
+}
+
+// read the destination back through the same GPU path (hash only) and compare with the source's hashes
+int verify_destination(const Manifest& man, const FileIO& io, const std::vector<BlockRef>& blocks,
+                       const std::vector<uint64_t>& hashes, const vmig_opts& o, vmig_stats* st)
+{
+    FileIO vio;
+    vio.hash_only = true;
+    vio.direct = io.direct;          // O_DIRECT re-read: what is verified is what the device holds, not the page cache
+    vio.cufile = io.cufile;
+    int rc = vio.setup(io.dst_root, man);
+    if (rc) return rc;
+    std::vector<BlockRef> vblocks = blocks;
+    for (auto& b : vblocks) { b.prior_hash = 0; b.prior_valid = 0; }
+    std::vector<uint64_t> vh(man.n_blocks, 0);
+    vmig_stats vst; memset(&vst, 0, sizeof vst);
+    rc = run_blocks(vblocks, &vio, false, true, o, vh.data(), &vst);
+    if (rc) return rc;
+    st->kernel_launches += vst.kernel_launches; st->ms_kernel += vst.ms_kernel; st->bytes_h2d += vst.bytes_h2d;
+    for (auto& b : vblocks)
+        if (vh[b.table_idx] != hashes[b.table_idx])
+            return fail(VMIG_EVERIFY, "verify: %s block %llu hashes %016llx in the destination, %016llx in the source",
+                        man.files[b.file].rel.c_str(), (unsigned long long)(b.file_off / o.block_bytes),
+                        (unsigned long long)vh[b.table_idx], (unsigned long long)hashes[b.table_idx]);
+    if (o.flags & VMIG_F_PRUNE) {               // the destination's entry set must now equal the source's
+        uint64_t extras = 0;
+        rc = prune_extras(io.dst_root, man, true, &extras); if (rc) return rc;
+        if (extras) return fail(VMIG_EVERIFY, "verify: %llu destination entries are not in the source after pruning", (unsigned long long)extras);
+    }
+    return VMIG_OK;
+}
+
+int store_table(const char* out_path, const Manifest& man, const FileIO& io, const std::vector<uint64_t>& hashes, uint32_t block_bytes)
+{
+    BlockTable t; t.block_bytes = block_bytes; t.algo = 1;
+    t.files.reserve(man.files.size());
+    for (uint32_t f = 0; f < man.files.size(); f++) {
+        const Entry& e = man.files[f];
+        const bool own = e.hardlink_of < 0 && (e.n_blocks || !io.hash_only);         // hard-linked paths are never patched in place
+        t.files.push_back({e.rel, e.size, e.first_block, own ? io.fs[f].id_ino : 0, own ? io.fs[f].id_ctime_ns : 0});
+    }
+    t.hashes = hashes;
+    return table_store(out_path, t);
+}
+
+// the old volume's data is about to be unlinked: deferred write-back errors (ENOSPC / EIO on delayed allocation, network
+// filesystems) must surface first.  A no-op on tmpfs; one flush on a disk.
+int flush_and_remove_source(const std::string& src, const std::string& dst, const Manifest& man)
+{
+    int dfd = open(dst.c_str(), O_RDONLY | O_DIRECTORY | O_CLOEXEC);
+    if (dfd < 0) return fail(VMIG_EIO, "open %s: %s", dst.c_str(), errno_str(errno).c_str());
+    const int sr = syncfs(dfd); const int se = errno;
+    close(dfd);
+    if (sr != 0) return fail(VMIG_EIO, "syncfs %s: %s (source left in place)", dst.c_str(), errno_str(se).c_str());
+    return remove_source(src, man);
+}
+
+int migrate_tree_impl(const char* src_dir, const char* dst_dir, const char* prior_path, const char* out_path,
+                      const vmig_opts* opts_in, vmig_stats* stats_out)
+{
+    vmig_stats st; memset(&st, 0, sizeof st);
+    const uint64_t t_begin = now_ns();
+    vmig_opts o;
+    int rc = check_args(src_dir, dst_dir, opts_in, &o);
+    if (rc) return rc;
+    const bool hash_only = (o.flags & VMIG_F_HASH_ONLY) != 0;
+    const std::string src(src_dir), dst(dst_dir ? dst_dir : "");
+
+    Manifest man;
+    uint64_t t0 = now_ns();
+    rc = walk_tree(src, o.block_bytes, (o.flags & VMIG_F_SKIP_HIDDEN_TOPDIRS) != 0, &man);
+    if (rc) return rc;
+    st.ns_walk = now_ns() - t0;
+
+    t0 = now_ns();
+    BlockTable prior; const bool has_prior = prior_path && *prior_path && !hash_only;
+    if (has_prior) {
+        rc = table_load(prior_path, &prior);
+        if (rc) return rc;
+        if (prior.block_bytes != o.block_bytes) return fail(VMIG_ETABLE, "prior table block size %u != %u", prior.block_bytes, o.block_bytes);
+    }
+    FileIO io;
+    io.dst_root = dst; io.pol = default_meta_policy(o.flags); io.hash_only = hash_only;
+    io.corrupt_block = env_long("VMIG_CORRUPT_BLOCK", -1);
+    io.direct = (o.flags & VMIG_F_DIRECT_IO) != 0;
+    io.cufile = (o.flags & VMIG_F_CUFILE) != 0;
+    rc = io.setup(src, man);
+    if (rc) return rc;
+    std::vector<uint64_t> hashes(man.n_blocks, 0);
+    std::vector<BlockRef> blocks;
+    plan_blocks(man, has_prior ? &prior : nullptr, o.block_bytes, io, &blocks, &st.files_untrusted);
     st.ns_plan = now_ns() - t0;
 
     // VMIG_F_PRUNE runs first: what it removes is by definition not in the source, a directory sitting where the source
@@ -469,7 +545,7 @@ int migrate_tree_impl(const char* src_dir, const char* dst_dir, const char* prio
     t0 = now_ns();
     rc = run_blocks(blocks, &io, has_prior, hash_only, o, hashes.data(), &st);
     st.ns_data = now_ns() - t0;
-    if (rc) { std::string keep = last_error_cstr(); io.close_all(man.files.size()); set_last_error_str(keep); return rc; }
+    if (rc) return rc;
 
     t0 = now_ns();
     for (auto& e : man.files)                      // hard-linked paths share their primary's hashes
@@ -478,85 +554,19 @@ int migrate_tree_impl(const char* src_dir, const char* dst_dir, const char* prio
             for (uint64_t r = 0; r < e.n_blocks; r++) hashes[e.first_block + r] = hashes[p.first_block + r];
         }
     if (!hash_only) {
-        for (auto& e : man.files) {                // empty regular files carry no blocks
-            if (e.hardlink_of >= 0 || e.n_blocks) continue;
-            const std::string p = pjoin(dst, e.rel);
-            bool was_dir = false;
-            rc = unlink_if_exists(p, &was_dir); if (rc) return rc;
-            if (was_dir) return fail(VMIG_EIO, "%s: a directory is in the way of a regular file", p.c_str());
-            int fd = open(p.c_str(), O_WRONLY | O_CREAT | O_EXCL | O_CLOEXEC | O_NOFOLLOW, 0600);
-            if (fd < 0) return fail(VMIG_EIO, "create %s: %s", p.c_str(), errno_str(errno).c_str());
-            rc = apply_file_meta(fd, p, e, io.pol);
-            struct stat ids;
-            if (!rc && fstat(fd, &ids) == 0) {
-                FileIO::FS& s = io.fs[&e - &man.files[0]];
-                s.id_ino = (uint64_t)ids.st_ino; s.id_ctime_ns = (int64_t)ids.st_ctim.tv_sec * 1000000000ll + ids.st_ctim.tv_nsec;
-            }
-            close(fd);
-            if (rc) return rc;
-        }
-        rc = replay_metadata(dst, man, io.pol, &st.symlinks, &st.hardlinks, &st.specials);
+        rc = create_empty_files(man, io);
+        if (!rc) rc = replay_metadata(dst, man, io.pol, &st.symlinks, &st.hardlinks, &st.specials);
         if (rc) return rc;
     }
     st.ns_meta = now_ns() - t0;
 
-    if ((o.flags & VMIG_F_VERIFY) && !hash_only) {
-        // read the destination back through the same GPU path (hash only) and compare block tables
-        FileIO vio;
-        vio.src_root = dst; vio.dst_root = dst; vio.m = &man; vio.pol = io.pol; vio.hash_only = true;
-        vio.direct = io.direct;          // O_DIRECT re-read: what is verified is what the device holds, not the page cache
-        vio.cufile = io.cufile;
-        vio.fs.reset(new FileIO::FS[man.files.size() ? man.files.size() : 1]);
-        rc = vio.open_root(); if (rc) return rc;
-        for (uint32_t f = 0; f < man.files.size(); f++) {
-            const Entry& e = man.files[f];
-            if (e.hardlink_of >= 0 || e.n_blocks == 0) continue;
-            vio.fs[f].reads_left.store((uint32_t)e.n_blocks); vio.fs[f].blocks_left.store((uint32_t)e.n_blocks);
-        }
-        std::vector<BlockRef> vblocks = blocks;
-        for (auto& b : vblocks) { b.prior_hash = 0; b.prior_valid = 0; }
-        std::vector<uint64_t> vh(man.n_blocks, 0);
-        vmig_stats vst; memset(&vst, 0, sizeof vst);
-        rc = run_blocks(vblocks, &vio, false, true, o, vh.data(), &vst);
-        if (rc) { std::string keep = last_error_cstr(); vio.close_all(man.files.size()); set_last_error_str(keep); return rc; }
-        st.kernel_launches += vst.kernel_launches; st.ms_kernel += vst.ms_kernel; st.bytes_h2d += vst.bytes_h2d;
-        for (auto& b : vblocks)
-            if (vh[b.table_idx] != hashes[b.table_idx])
-                return fail(VMIG_EVERIFY, "verify: %s block %llu hashes %016llx in the destination, %016llx in the source",
-                            man.files[b.file].rel.c_str(), (unsigned long long)(b.file_off / o.block_bytes),
-                            (unsigned long long)vh[b.table_idx], (unsigned long long)hashes[b.table_idx]);
-        if (o.flags & VMIG_F_PRUNE) {               // the destination's entry set must now equal the source's
-            uint64_t extras = 0;
-            rc = prune_extras(dst, man, true, &extras); if (rc) return rc;
-            if (extras) return fail(VMIG_EVERIFY, "verify: %llu destination entries are not in the source after pruning", (unsigned long long)extras);
-        }
-    }
+    if ((o.flags & VMIG_F_VERIFY) && !hash_only) { rc = verify_destination(man, io, blocks, hashes, o, &st); if (rc) return rc; }
 
     t0 = now_ns();
-    if (out_path && *out_path) {
-        BlockTable t; t.block_bytes = o.block_bytes; t.algo = 1;
-        t.files.reserve(man.files.size());
-        for (uint32_t f = 0; f < man.files.size(); f++) {
-            const Entry& e = man.files[f];
-            const bool own = e.hardlink_of < 0 && (e.n_blocks || !hash_only);         // hard-linked paths are never patched in place
-            t.files.push_back({e.rel, e.size, e.first_block, own ? io.fs[f].id_ino : 0, own ? io.fs[f].id_ctime_ns : 0});
-        }
-        t.hashes = hashes;
-        rc = table_store(out_path, t);
-        if (rc) return rc;
-    }
+    if (out_path && *out_path) { rc = store_table(out_path, man, io, hashes, o.block_bytes); if (rc) return rc; }
     st.ns_table = now_ns() - t0;
 
-    if ((o.flags & VMIG_F_MOVE_SRC) && !hash_only) {
-        // the old volume's data is about to be unlinked: deferred write-back errors (ENOSPC / EIO on delayed
-        // allocation, network filesystems) must surface first.  A no-op on tmpfs; one flush on a disk.
-        int dfd = open(dst.c_str(), O_RDONLY | O_DIRECTORY | O_CLOEXEC);
-        if (dfd < 0) return fail(VMIG_EIO, "open %s: %s", dst.c_str(), errno_str(errno).c_str());
-        const int sr = syncfs(dfd); const int se = errno;
-        close(dfd);
-        if (sr != 0) return fail(VMIG_EIO, "syncfs %s: %s (source left in place)", dst.c_str(), errno_str(se).c_str());
-        rc = remove_source(src, man); if (rc) return rc;
-    }
+    if ((o.flags & VMIG_F_MOVE_SRC) && !hash_only) { rc = flush_and_remove_source(src, dst, man); if (rc) return rc; }
 
     st.files_direct = io.n_direct.load();
     st.bytes_total = man.bytes_total; st.blocks_total = man.n_blocks;
@@ -629,11 +639,12 @@ int vmig_migrate_buffer(const void* src, void* dst, uint64_t nbytes, const uint6
 {
     vmig_stats st; memset(&st, 0, sizeof st);
     const uint64_t t0 = now_ns();
-    vmig_opts o = norm_opts(opts);
+    vmig_opts o;
+    int rc = norm_opts(opts, &o);
+    if (rc) return rc;
     const bool hash_only = (o.flags & VMIG_F_HASH_ONLY) != 0;
     if (!src || (!dst && !hash_only)) return fail(VMIG_EINVAL, "null buffer");
-    if ((o.block_bytes & 4095u) || o.block_bytes > pipe_slot_bytes()) return fail(VMIG_EINVAL, "bad block_bytes %u", o.block_bytes);
-    std::vector<DeviceInfo> devs; int rc = ctx_select(o.gpu_mask, &devs); if (rc) return rc;
+    std::vector<DeviceInfo> devs; rc = ctx_select(o.gpu_mask, &devs); if (rc) return rc;
     const uint64_t nb = (nbytes + o.block_bytes - 1) / o.block_bytes;
     std::vector<BlockRef> blocks(nb);
     const bool has_prior = prior_hashes != nullptr && prior_valid != nullptr;
@@ -675,7 +686,6 @@ int vmig_hash_blocks(int gpu, const void* host_buf, const uint64_t* offs, const 
 
 // ---------------------------------------------------------------------------------------------
 // host<->HBM link probe
-#define CU_API(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { cudaGetLastError(); return fail(e__ == cudaErrorMemoryAllocation ? VMIG_ENOMEM : VMIG_ECUDA, "%s: %s", #call, cudaGetErrorString(e__)); } } while (0)
 
 static int link_probe_here(int gpu, uint64_t bytes, double* gbs)
 {

@@ -1,6 +1,7 @@
 // vmig_common.h -- shared host-side helpers of libvmig (errors, timing, small utilities).
 #pragma once
 #include <stdint.h>
+#include <sys/types.h>
 #include <string>
 #include <chrono>
 #include <cstdarg>
@@ -32,6 +33,28 @@ inline int fail(int code, const char* fmt, ...) {
 inline std::string errno_str(int e) { char b[128]; return std::string(strerror_r(e, b, sizeof b)); }
 
 inline uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
+
+// Moves the `len` bytes of a block at file offset `file_off` through op(pos, n) -> bytes moved, or a negative VMIG_E*
+// code, for the n bytes at offset pos inside the block.  `name` and `file_off` only label the error.
+//   align == 0: buffered I/O; a short transfer resumes at the exact byte.
+//   align != 0 (an O_DIRECT descriptor: buffer, offset and length in whole sectors): every transfer runs to the
+//     rounded-up end of the block, so the file's short last block reads or writes past EOF and simply moves fewer
+//     bytes; a short transfer inside the block resumes from the last sector boundary it reached.
+// A transfer that moves nothing new fails with `stuck` (VMIG_ESRCCHANGED for a source that shrank under a reader).
+template <class Op>
+inline int transfer_block(const char* name, uint64_t file_off, size_t len, size_t align, int stuck, Op&& op) {
+    const size_t want = align ? (size_t)align_up(len, align) : len;
+    size_t done = 0;
+    while (done < len) {
+        const size_t pos = align ? (done & ~(align - 1)) : done;
+        const ssize_t r = op(pos, want - pos);
+        if (r < 0) return (int)r;
+        if (r == 0 || pos + (size_t)r <= done)
+            return fail(stuck, "%s: no progress after %zu of %zu bytes at offset %llu", name, done, len, (unsigned long long)file_off);
+        done = pos + (size_t)r;
+    }
+    return VMIG_OK;
+}
 
 long env_long(const char* name, long dflt);
 

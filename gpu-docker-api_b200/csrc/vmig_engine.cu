@@ -38,14 +38,6 @@ long env_long(const char* name, long dflt) {
     return end && *end == 0 ? r : dflt;
 }
 
-#define CU_TRY(call)                                                                                  \
-    do {                                                                                              \
-        cudaError_t e__ = (call);                                                                     \
-        if (e__ != cudaSuccess)                                                                       \
-            return fail(e__ == cudaErrorMemoryAllocation ? VMIG_ENOMEM : VMIG_ECUDA, "%s: %s", #call, \
-                        cudaGetErrorString(e__));                                                     \
-    } while (0)
-
 // ---------------------------------------------------------------------------------------------
 // tunables (env, read once per process)
 static constexpr uint32_t kMaxBatchBlocks = 4096;
@@ -114,7 +106,7 @@ static int ring_alloc(uint8_t** out, size_t bytes, size_t* mapped)
             munmap(a, len);
         }
     }
-    CU_TRY(cudaHostAlloc((void**)out, bytes, cudaHostAllocPortable));
+    CU_API(cudaHostAlloc((void**)out, bytes, cudaHostAllocPortable));
     memset(*out, 0, bytes);
     return VMIG_OK;
 }
@@ -155,7 +147,7 @@ int Pipe::create_here(const DeviceInfo& d)
 {
     load_tunables();
     dev = d; slot_bytes = g_slot_bytes;
-    CU_TRY(cudaSetDevice(d.dev));
+    CU_API(cudaSetDevice(d.dev));
     slots.resize(g_slots);
     const size_t cap = (size_t)slot_bytes + kTailPad;
     // Which socket's DRAM holds the rings (first touch decides).  0 = the GPU's socket, 1 = the other socket(s),
@@ -177,19 +169,19 @@ int Pipe::create_here(const DeviceInfo& d)
         { int rc = ring_alloc(&s.h_out, cap, &s.out_mapped); if (rc) return rc; }
         bind_thread(d);
         slot_idx++;
-        CU_TRY(cudaMalloc((void**)&s.d_buf, cap));
-        CU_TRY(cudaMemset(s.d_buf, 0, cap));
-        CU_TRY(cudaHostAlloc((void**)&s.h_desc, kDescBytes, cudaHostAllocPortable));
-        CU_TRY(cudaMalloc((void**)&s.d_desc, kDescBytes));
-        CU_TRY(cudaHostAlloc((void**)&s.h_res, kResBytes, cudaHostAllocPortable));
-        CU_TRY(cudaMalloc((void**)&s.d_res, kResBytes));
-        CU_TRY(cudaMalloc((void**)&s.d_counter, 256));
-        CU_TRY(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-        CU_TRY(cudaEventCreate(&s.ev_k0)); CU_TRY(cudaEventCreate(&s.ev_k1));
-        CU_TRY(cudaEventCreateWithFlags(&s.ev_hash, cudaEventDisableTiming));
-        CU_TRY(cudaEventCreateWithFlags(&s.ev_d2h, cudaEventDisableTiming));
+        CU_API(cudaMalloc((void**)&s.d_buf, cap));
+        CU_API(cudaMemset(s.d_buf, 0, cap));
+        CU_API(cudaHostAlloc((void**)&s.h_desc, kDescBytes, cudaHostAllocPortable));
+        CU_API(cudaMalloc((void**)&s.d_desc, kDescBytes));
+        CU_API(cudaHostAlloc((void**)&s.h_res, kResBytes, cudaHostAllocPortable));
+        CU_API(cudaMalloc((void**)&s.d_res, kResBytes));
+        CU_API(cudaMalloc((void**)&s.d_counter, 256));
+        CU_API(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
+        CU_API(cudaEventCreate(&s.ev_k0)); CU_API(cudaEventCreate(&s.ev_k1));
+        CU_API(cudaEventCreateWithFlags(&s.ev_hash, cudaEventDisableTiming));
+        CU_API(cudaEventCreateWithFlags(&s.ev_d2h, cudaEventDisableTiming));
     }
-    CU_TRY(cudaDeviceSynchronize());
+    CU_API(cudaDeviceSynchronize());
     return VMIG_OK;
 }
 void Pipe::destroy()
@@ -628,18 +620,18 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
             h_offs[i] = slot_off[b->b0 + i]; h_prior[i] = r.prior_hash; h_lens[i] = r.len; h_valid[i] = r.prior_valid;
         }
         const size_t desc_bytes = (size_t)n * 21;
-        CU_TRY(cudaMemcpyAsync(sl.d_desc, sl.h_desc, desc_bytes, cudaMemcpyHostToDevice, sl.stream));
+        CU_API(cudaMemcpyAsync(sl.d_desc, sl.h_desc, desc_bytes, cudaMemcpyHostToDevice, sl.stream));
         uint64_t h2d = 0;
         if (direct_src) {
             for (uint32_t i = 0; i < n; i++) {
                 const BlockRef& r = blocks[b->b0 + i];
                 if (!r.len) continue;
-                CU_TRY(cudaMemcpyAsync(sl.d_buf + slot_off[b->b0 + i], io->pinned_src(r), r.len, cudaMemcpyHostToDevice, sl.stream));
+                CU_API(cudaMemcpyAsync(sl.d_buf + slot_off[b->b0 + i], io->pinned_src(r), r.len, cudaMemcpyHostToDevice, sl.stream));
                 h2d += r.len;
             }
         } else {
             // (GPUDirect Storage backends already put the bytes into the HBM slot on the reader threads)
-            if (!dev_src) CU_TRY(cudaMemcpyAsync(sl.d_buf, sl.h_in, b->bytes_used, cudaMemcpyHostToDevice, sl.stream));
+            if (!dev_src) CU_API(cudaMemcpyAsync(sl.d_buf, sl.h_in, b->bytes_used, cudaMemcpyHostToDevice, sl.stream));
             for (uint32_t i = 0; i < n; i++) h2d += blocks[b->b0 + i].len;
         }
         HashLaunch a;
@@ -648,25 +640,25 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
         a.n = n; a.hashes = (uint64_t*)sl.d_res; a.changed = (uint8_t*)(a.hashes + n);
         a.work_counter = sl.d_counter;
         if (!has_prior) { a.prior = nullptr; a.prior_valid = nullptr; }
-        CU_TRY(cudaEventRecord(sl.ev_k0, sl.stream));
-        CU_TRY(launch_xxh64_blocks(a, pipe->dev.sm_count, sl.stream));
-        CU_TRY(cudaEventRecord(sl.ev_k1, sl.stream));
-        CU_TRY(cudaMemcpyAsync(sl.h_res, sl.d_res, (size_t)n * 9, cudaMemcpyDeviceToHost, sl.stream));
-        CU_TRY(cudaEventRecord(sl.ev_hash, sl.stream));
+        CU_API(cudaEventRecord(sl.ev_k0, sl.stream));
+        CU_API(launch_xxh64_blocks(a, pipe->dev.sm_count, sl.stream));
+        CU_API(cudaEventRecord(sl.ev_k1, sl.stream));
+        CU_API(cudaMemcpyAsync(sl.h_res, sl.d_res, (size_t)n * 9, cudaMemcpyDeviceToHost, sl.stream));
+        CU_API(cudaEventRecord(sl.ev_hash, sl.stream));
         uint64_t d2h = 0;
         if (!has_prior && !hash_only && !dev_dst) {       // every block survives: stream it back right away
             if (direct_dst) {
                 for (uint32_t i = 0; i < n; i++) {
                     const BlockRef& r = blocks[b->b0 + i];
                     if (!r.len) continue;
-                    CU_TRY(cudaMemcpyAsync(io->pinned_dst(r), sl.d_buf + slot_off[b->b0 + i], r.len, cudaMemcpyDeviceToHost, sl.stream));
+                    CU_API(cudaMemcpyAsync(io->pinned_dst(r), sl.d_buf + slot_off[b->b0 + i], r.len, cudaMemcpyDeviceToHost, sl.stream));
                     d2h += r.len;
                 }
             } else {
-                CU_TRY(cudaMemcpyAsync(sl.h_out, sl.d_buf, b->bytes_used, cudaMemcpyDeviceToHost, sl.stream));
+                CU_API(cudaMemcpyAsync(sl.h_out, sl.d_buf, b->bytes_used, cudaMemcpyDeviceToHost, sl.stream));
                 d2h = h2d;
             }
-            CU_TRY(cudaEventRecord(sl.ev_d2h, sl.stream));
+            CU_API(cudaEventRecord(sl.ev_d2h, sl.stream));
         }
         std::lock_guard<std::mutex> lk(stat_mu);
         stats->bytes_h2d += h2d; stats->bytes_d2h += d2h; stats->kernel_launches += 1;
@@ -688,8 +680,8 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
     auto after_hash = [&](Batch* b) -> int {
         Slot& sl = pipe->slots[b->slot];
         const uint32_t n = (uint32_t)(b->b1 - b->b0);
-        CU_TRY(cudaEventSynchronize(sl.ev_hash));
-        float ms = 0; CU_TRY(cudaEventElapsedTime(&ms, sl.ev_k0, sl.ev_k1));
+        CU_API(cudaEventSynchronize(sl.ev_hash));
+        float ms = 0; CU_API(cudaEventElapsedTime(&ms, sl.ev_k0, sl.ev_k1));
         const uint64_t* h_hash = (const uint64_t*)sl.h_res; const uint8_t* h_changed = (const uint8_t*)(h_hash + n);
         b->survive.assign(n, 1);
         uint64_t skipped = 0, d2h = 0;
@@ -707,15 +699,15 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
                 if (!b->survive[i] || !blocks[b->b0 + i].len) { i++; continue; }
                 if (direct_dst) {
                     const BlockRef& r = blocks[b->b0 + i];
-                    CU_TRY(cudaMemcpyAsync(io->pinned_dst(r), sl.d_buf + slot_off[b->b0 + i], r.len, cudaMemcpyDeviceToHost, sl.stream));
+                    CU_API(cudaMemcpyAsync(io->pinned_dst(r), sl.d_buf + slot_off[b->b0 + i], r.len, cudaMemcpyDeviceToHost, sl.stream));
                     d2h += r.len; i++; continue;
                 }
                 uint32_t j = i; size_t start = slot_off[b->b0 + i], end = start;
                 while (j < n && b->survive[j]) { end = slot_off[b->b0 + j] + blocks[b->b0 + j].len; d2h += blocks[b->b0 + j].len; j++; }
-                CU_TRY(cudaMemcpyAsync(sl.h_out + start, sl.d_buf + start, end - start, cudaMemcpyDeviceToHost, sl.stream));
+                CU_API(cudaMemcpyAsync(sl.h_out + start, sl.d_buf + start, end - start, cudaMemcpyDeviceToHost, sl.stream));
                 i = j;
             }
-            CU_TRY(cudaEventRecord(sl.ev_d2h, sl.stream));
+            CU_API(cudaEventRecord(sl.ev_d2h, sl.stream));
         }
         std::lock_guard<std::mutex> lk(stat_mu);
         stats->ms_kernel += ms; stats->blocks_skipped += skipped; stats->bytes_d2h += d2h;

@@ -20,6 +20,18 @@
 
 namespace vmig {
 
+// Return VMIG_ENOMEM / VMIG_ECUDA from the enclosing function when a CUDA runtime call fails.  The runtime's last error
+// is cleared, so a later launch check on this thread (cudaGetLastError) does not report it a second time.
+#define CU_API(call)                                                                                  \
+    do {                                                                                              \
+        cudaError_t e__ = (call);                                                                     \
+        if (e__ != cudaSuccess) {                                                                     \
+            cudaGetLastError();                                                                       \
+            return fail(e__ == cudaErrorMemoryAllocation ? VMIG_ENOMEM : VMIG_ECUDA, "%s: %s", #call, \
+                        cudaGetErrorString(e__));                                                     \
+        }                                                                                             \
+    } while (0)
+
 struct BlockRef {
     uint32_t file;         // backend-defined (index of the file in the manifest; 0 for buffers)
     uint32_t len;          // bytes in this block (<= block_bytes; 0 allowed)

@@ -124,6 +124,18 @@ def test_writer_queue_invariants(tmp_path):
     assert r.returncode == 0 and "sched unit ok" in r.stdout, r.stdout + r.stderr
 
 
+def test_block_transfer_loop(tmp_path):
+    """csrc/vmig_common.h transfer_block alone (no GPU): buffered resume at the exact byte, O_DIRECT resume from the
+    sector boundary, a short last block, no progress and a failing transfer -- with a scripted fake in place of the I/O."""
+    import subprocess
+    exe = tmp_path / "xfer_unit"
+    csrc = ROOT / "gpu-docker-api_b200" / "csrc"
+    subprocess.run(["g++", "-std=c++17", "-O2", "-Wall", "-Werror", "-I", str(csrc), str(ROOT / "tests" / "xfer_unit.cpp"),
+                    "-o", str(exe)], check=True)
+    r = subprocess.run([str(exe)], capture_output=True, text=True, timeout=60)
+    assert r.returncode == 0 and "xfer unit ok" in r.stdout, r.stdout + r.stderr
+
+
 def test_struct_layouts_match_header(vm):
     assert ctypes.sizeof(vm.Opts) == 32
     assert ctypes.sizeof(vm.Stats) == 18 * 8 + 8 + 8 + 24
