@@ -154,19 +154,20 @@ public:
         }
         *out = fd; return VMIG_OK;
     }
-    // O_DIRECT: buffer, offset and length in whole sectors (the slot layout leaves the room; the device DMAs straight
-    // into the pinned ring)
-    int read_block(const BlockRef& b, uint8_t* dst) override {
+    // O_DIRECT: buffer, offset and length in whole sectors (pieces are whole sectors; the device DMAs straight into the
+    // reader's pinned piece).  The source is closed after the last piece of its last block.
+    int read_block(const BlockRef& b, size_t off, size_t len, uint8_t* dst) override {
         int fd; int rc = open_src(b.file, &fd);
         if (rc) return rc;
         FS& s = fs[b.file];
         const char* name = m->files[b.file].rel.c_str();
-        rc = transfer_block(name, b.file_off, b.len, s.s_direct ? kSector : 0, VMIG_ESRCCHANGED, [&](size_t pos, size_t n) -> ssize_t {
+        const uint64_t at = b.file_off + off;
+        rc = transfer_block(name, at, len, s.s_direct ? kSector : 0, VMIG_ESRCCHANGED, [&](size_t pos, size_t n) -> ssize_t {
             ssize_t r;
-            while ((r = pread(fd, dst + pos, n, (off_t)(b.file_off + pos))) < 0 && errno == EINTR) {}
+            while ((r = pread(fd, dst + pos, n, (off_t)(at + pos))) < 0 && errno == EINTR) {}
             return r < 0 ? fail(VMIG_EIO, "pread %s: %s", name, errno_str(errno).c_str()) : r;
         });
-        if (!rc && s.reads_left.fetch_sub(1) == 1) close_src(s, fd);
+        if (!rc && off + len == b.len && s.reads_left.fetch_sub(1) == 1) close_src(s, fd);
         return rc;
     }
     void close_src(FS& s, int fd) {
@@ -252,7 +253,7 @@ class MemIO : public BlockIO {
 public:
     const uint8_t* src = nullptr; uint8_t* dst = nullptr;
     bool src_pinned = false, dst_pinned = false;
-    int read_block(const BlockRef& b, uint8_t* d) override { if (b.len) memcpy(d, src + b.file_off, b.len); return VMIG_OK; }
+    int read_block(const BlockRef& b, size_t off, size_t len, uint8_t* d) override { if (len) memcpy(d, src + b.file_off + off, len); return VMIG_OK; }
     int write_block(const BlockRef& b, const uint8_t* s) override { if (b.len) memcpy(dst + b.file_off, s, b.len); return VMIG_OK; }
     uint32_t write_key(const BlockRef& b) override { return (uint32_t)b.table_idx; }
     const uint8_t* pinned_src(const BlockRef& b) override { return src_pinned ? src + b.file_off : nullptr; }

@@ -56,6 +56,26 @@ inline int transfer_block(const char* name, uint64_t file_off, size_t len, size_
     return VMIG_OK;
 }
 
+// Readers stage a slot in windows of `piece` bytes: window w is slot bytes [w * piece, (w + 1) * piece), filled in one
+// pinned piece and copied to the GPU in one go, so that consecutive small blocks share a copy.  A block at slot offset
+// `at` is read in the parts that fall in successive windows; an empty block is one empty part, so that every block is
+// read exactly once whatever its length.
+struct Piece {
+    size_t window;   // index of the window
+    size_t off;      // offset of the part inside the block
+    size_t len;      // bytes of the block in this part
+    size_t io_len;   // what the read asks for: len rounded up to whole sectors when align != 0 (O_DIRECT), which the
+                     // file's short last block reads past EOF.  With `at` and `piece` whole sectors, the read ends
+                     // inside its window
+};
+inline size_t piece_count(size_t at, size_t len, size_t piece) { return len ? (at + len - 1) / piece - at / piece + 1 : 1; }
+inline Piece block_piece(size_t at, size_t len, size_t piece, size_t align, size_t k) {
+    const size_t w = at / piece + k, w0 = w * piece, w1 = w0 + piece;
+    const size_t start = at > w0 ? at : w0, end = at + len < w1 ? at + len : w1;
+    const size_t n = end > start ? end - start : 0;
+    return {w, start - at, n, align ? (size_t)align_up(n, align) : n};
+}
+
 long env_long(const char* name, long dflt);
 
 }  // namespace vmig

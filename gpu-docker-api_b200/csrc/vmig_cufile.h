@@ -1,5 +1,5 @@
 // vmig_cufile.h -- GPUDirect Storage (cuFile) ingest, SURVEY.md §8f row N4: source blocks go from the file straight into
-// the HBM staging slot (no pinned IN ring, no separate H2D copy).  libcufile is dlopen()ed at first use, so libvmig has
+// the HBM staging slot (no pinned pieces, no separate H2D copy).  libcufile is dlopen()ed at first use, so libvmig has
 // no link-time dependency on it; with the nvidia-fs kernel module the read is a DMA from the NVMe into HBM, without it
 // libcufile's compatibility mode (POSIX read + its own bounce buffers) gives the same bytes.
 // Deployment the row targets: Docker root on local xfs/LVM (reference docs/volume/volume-size-scale-en.md:5-21).

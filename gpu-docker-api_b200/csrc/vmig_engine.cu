@@ -58,7 +58,6 @@ uint32_t pipe_slot_bytes() { load_tunables(); return g_slot_bytes; }
 // ---------------------------------------------------------------------------------------------
 // slot / pipe
 struct Slot {
-    uint8_t* h_in = nullptr;    // pinned, slot_bytes + pad
     uint8_t* h_out = nullptr;   // pinned, slot_bytes + pad
     uint8_t* d_buf = nullptr;   // HBM,    slot_bytes + pad
     uint8_t* h_desc = nullptr;  // pinned: packed [offs u64][prior u64][lens u32][valid u8] for n blocks
@@ -68,14 +67,14 @@ struct Slot {
     uint32_t* d_counter = nullptr;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr, ev_hash = nullptr, ev_d2h = nullptr;
-    size_t in_mapped = 0, out_mapped = 0;   // > 0: ring is an mmap'ed huge-page region registered with CUDA
+    size_t out_mapped = 0;                  // > 0: ring is an mmap'ed huge-page region registered with CUDA
     bool cf_registered = false;             // d_buf is registered with cuFile (GPUDirect Storage backends)
 };
 
 // Staging rings: 2 MiB-aligned anonymous memory with MADV_HUGEPAGE, faulted in, then page-locked
 // with cudaHostRegister -- the kernel's copy_to/from_user and the DMA engines then walk 16 huge
-// pages per 32 MiB slot instead of 8 192 small ones.  Falls back to cudaHostAlloc (VMIG_HUGE=0, or
-// if the mapping / registration fails).
+// pages per 32 MiB slot instead of 8 192 small ones.  The OUT ring has one per slot, the readers' pieces one per pipe.
+// Falls back to cudaHostAlloc (VMIG_HUGE=0, or if the mapping / registration fails).
 static int ring_alloc(uint8_t** out, size_t bytes, size_t* mapped)
 {
     *mapped = 0;
@@ -118,22 +117,38 @@ static void ring_free(uint8_t* p, size_t mapped)
 static constexpr size_t kDescBytes = (size_t)kMaxBatchBlocks * (8 + 8 + 4 + 1) + 64;
 static constexpr size_t kResBytes  = (size_t)kMaxBatchBlocks * (8 + 1) + 64;
 
+// Reader staging: each reader owns kPieces pinned pieces of kPieceBytes and copies each one into the HBM slot as soon as
+// it is filled, so a staged byte is still in the CPU's cache when the DMA reads it (a 32 MiB slot staged whole is written
+// back to DRAM and read from there again).  The probe loop measured 22.2-22.9 GiB/s with 4 x 1 MiB private pieces against
+// 12.3-13.9 with pieces rotating through a 512 MiB ring (profiles/r01_piece_probe.txt); 16 pieces per reader gained
+// nothing over 4 (profiles/r03_piece_variants.txt).  Pieces are whole sectors, so the rounded-up O_DIRECT read of a
+// file's short last block ends inside its piece.
+static constexpr uint32_t kPieces = 4, kPieceBytes = 1u << 20;
+static_assert(kPieceBytes % 4096 == 0, "an O_DIRECT piece is whole sectors");
+struct PieceReader {
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev[kPieces] = {};     // the last copy out of each piece
+};
+
 class Pipe {
 public:
     DeviceInfo dev;
     uint32_t slot_bytes = 0;
     std::vector<Slot> slots;
+    uint8_t* pieces = nullptr;        // readers.size() x kPieces x kPieceBytes, pinned
+    size_t pieces_mapped = 0;
+    std::vector<PieceReader> readers;
     int create(const DeviceInfo& d);
     int create_here(const DeviceInfo& d);
+    int reserve_readers(uint32_t n);
     void destroy();
 };
 
 static void bind_thread(const DeviceInfo& d);
 static void bind_thread_complement(const DeviceInfo& d);
 
-// The pinned rings are allocated and first-touched by a thread bound to the GPU's NUMA-local
-// CPUs, so that staging copies and both DMA directions stay on the GPU's socket (on the 2-socket
-// bench box a ring on the far socket sends every byte across UPI four times).
+// A pipe is created by a thread bound to the GPU's NUMA-local CPUs, so that what it first-touches stays on the GPU's
+// socket; only the OUT ring is placed on purpose (create_here).
 int Pipe::create(const DeviceInfo& d)
 {
     int rc = VMIG_OK; std::string msg;
@@ -150,12 +165,9 @@ int Pipe::create_here(const DeviceInfo& d)
     CU_API(cudaSetDevice(d.dev));
     slots.resize(g_slots);
     const size_t cap = (size_t)slot_bytes + kTailPad;
-    // Which socket's DRAM holds the rings (first touch decides).  0 = the GPU's socket, 1 = the other socket(s),
-    // 2 = alternate slot by slot.  Four of the six DRAM passes a migrated byte makes touch a ring (IN write, H2D read,
-    // D2H write, OUT read); with everything on the GPU's socket that socket's memory controllers carry ~75 % of the
-    // traffic while the other one idles.  The OUT ring defaults to the writers' side (VMIG_BIND_WRITERS=2 puts them on
-    // the other socket): the D2H DMA crosses UPI once, the writers then read it locally.
-    const long in_node = env_long("VMIG_RING_IN_NODE", 0);
+    // Which socket's DRAM holds the OUT ring (first touch decides).  0 = the GPU's socket, 1 = the other socket(s),
+    // 2 = alternate slot by slot.  It defaults to the writers' side (VMIG_BIND_WRITERS=2 puts them on the other socket):
+    // the D2H DMA crosses UPI once, the writers then read it locally.
     const long out_node = env_long("VMIG_RING_OUT_NODE", env_long("VMIG_BIND_WRITERS", 2) == 2 ? 1 : 0);      // +5..8 % end to end (profiles/r02_sweep_ring_placement.txt)
     auto place = [&](long mode, size_t idx) {
         const bool far = mode == 1 || (mode == 2 && (idx & 1));
@@ -163,8 +175,6 @@ int Pipe::create_here(const DeviceInfo& d)
     };
     size_t slot_idx = 0;
     for (auto& s : slots) {
-        place(in_node, slot_idx);
-        { int rc = ring_alloc(&s.h_in, cap, &s.in_mapped); if (rc) return rc; }
         place(out_node, slot_idx);
         { int rc = ring_alloc(&s.h_out, cap, &s.out_mapped); if (rc) return rc; }
         bind_thread(d);
@@ -184,13 +194,45 @@ int Pipe::create_here(const DeviceInfo& d)
     CU_API(cudaDeviceSynchronize());
     return VMIG_OK;
 }
+// Pieces for n readers.  The pool grows (up to the 64 readers a call may ask for) and is never shrunk; it is only replaced
+// between calls, when no copy reads it.  Allocated and first-touched on the GPU's socket, where the readers run.
+int Pipe::reserve_readers(uint32_t n)
+{
+    if (n <= readers.size() && pieces) return VMIG_OK;
+    int rc = VMIG_OK; std::string msg;
+    std::thread t([&] {
+        bind_thread(dev);
+        rc = [&]() -> int {
+            CU_API(cudaSetDevice(dev.dev));
+            ring_free(pieces, pieces_mapped); pieces = nullptr; pieces_mapped = 0;
+            { int r = ring_alloc(&pieces, (size_t)n * kPieces * kPieceBytes, &pieces_mapped); if (r) return r; }
+            while (readers.size() < n) {
+                readers.emplace_back();
+                PieceReader& pr = readers.back();
+                CU_API(cudaStreamCreateWithFlags(&pr.stream, cudaStreamNonBlocking));
+                for (auto& e : pr.ev) CU_API(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            }
+            return VMIG_OK;
+        }();
+        if (rc) msg = last_error_cstr();
+    });
+    t.join();
+    if (rc) set_last_error_str(msg);
+    return rc;
+}
 void Pipe::destroy()
 {
     cudaSetDevice(dev.dev);
+    for (auto& r : readers) {
+        if (r.stream) { cudaStreamSynchronize(r.stream); cudaStreamDestroy(r.stream); }
+        for (auto e : r.ev) if (e) cudaEventDestroy(e);
+    }
+    readers.clear();
+    ring_free(pieces, pieces_mapped); pieces = nullptr; pieces_mapped = 0;
     for (auto& s : slots) {
         if (s.stream) cudaStreamSynchronize(s.stream);
         if (s.cf_registered) { cufile_buf_deregister(s.d_buf); s.cf_registered = false; }
-        ring_free(s.h_in, s.in_mapped); ring_free(s.h_out, s.out_mapped); cudaFree(s.d_buf); cudaFreeHost(s.h_desc); cudaFree(s.d_desc);
+        ring_free(s.h_out, s.out_mapped); cudaFree(s.d_buf); cudaFreeHost(s.h_desc); cudaFree(s.d_desc);
         cudaFreeHost(s.h_res); cudaFree(s.d_res); cudaFree(s.d_counter);
         if (s.stream) cudaStreamDestroy(s.stream);
         if (s.ev_k0) cudaEventDestroy(s.ev_k0); if (s.ev_k1) cudaEventDestroy(s.ev_k1);
@@ -351,7 +393,7 @@ int ctx_acquire_pipes(const std::vector<DeviceInfo>& lane_devs, std::vector<Pipe
             to_create[k] = left; dp->n_pipes += left;        // reserved; created outside the lock
         }
     }
-    // new pipes of different lanes are created in parallel (page-locking 1 GiB of rings takes ~0.35 s each)
+    // new pipes of different lanes are created in parallel (each page-locks a 512 MiB OUT ring)
     int rc = VMIG_OK; std::string msg; std::mutex rmu;
     std::vector<std::thread> th;
     for (size_t i = 0; i < lane_devs.size(); i++) {
@@ -464,6 +506,11 @@ public:
         if (q.empty()) return false;
         *out = std::move(q.front()); q.pop_front(); return true;
     }
+    bool try_pop(T* out) {
+        std::lock_guard<std::mutex> lk(mu);
+        if (q.empty()) return false;
+        *out = std::move(q.front()); q.pop_front(); return true;
+    }
     void close() { { std::lock_guard<std::mutex> lk(mu); closed = true; } cv.notify_all(); }
 };
 
@@ -494,7 +541,7 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
     const long fail_block = env_long("VMIG_FAIL_BLOCK", -1);
     const bool bind_io = env_long("VMIG_BIND_IO", 1) != 0;      // reader/writer threads on the GPU's socket
     // writers default to the CPUs of the OTHER socket(s): destination pages then land in that socket's
-    // DRAM and the GPU-local socket (pinned rings, both DMA directions, the readers) is relieved of a
+    // DRAM and the GPU-local socket (the readers' pieces, both DMA directions, the readers) is relieved of a
     // third of the traffic (+15% end to end on the bench box); 1 = GPU-local CPUs, 0 = unbound
     const long bind_wr = env_long("VMIG_BIND_WRITERS", 2);
 
@@ -545,7 +592,7 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
     std::mutex done_mu; std::condition_variable done_cv; size_t batches_done = 0;
     std::mutex stat_mu;
 
-    std::atomic<uint64_t> rd_busy{0}, wr_busy{0}, slot_wait{0};
+    std::atomic<uint64_t> rd_busy{0}, wr_busy{0}, slot_wait{0}, piece_wait{0};
     const uint64_t lane_t0 = now_ns();
     auto finish_batch = [&](Batch* b) {
         b->t_done = now_ns();
@@ -558,6 +605,8 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
     // GPUDirect Storage backends: file <-> HBM slot without the pinned rings
     const bool dev_src = !direct_src && io->device_reads();
     const bool dev_dst = !hash_only && !direct_dst && io->device_writes();
+    const bool staged_src = !direct_src && !dev_src;       // read into the readers' pinned pieces
+    if (staged_src) { int rc = pipe->reserve_readers(n_readers); if (rc) { set_err(rc); return rc; } }
     if (dev_src || dev_dst) {
         cudaSetDevice(pipe->dev.dev);
         for (int s = 0; s < use_slots; s++) {
@@ -589,24 +638,96 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
         }
     });
 
-    // ---- stage 2: readers
+    // ---- stage 2: readers.  Reader t stages the slot window by window (vmig_common.h block_piece): it reads the parts of
+    // a task's blocks that fall in one window into one of its kPieces pieces, copies the filled range into the HBM slot on
+    // its own stream and records the piece's event.  A piece is refilled, and a task counts as read (so that its batch may
+    // be hashed, or its slot handed out again after an error), only once the copies out of it have completed.  The stream
+    // runs its copies in order, so one completed event vouches for every copy issued before it.  Two tasks never copy the
+    // same slot bytes: a copy spans the blocks' bytes only, never past the last one.
     std::vector<std::thread> readers;
     for (uint32_t t = 0; t < n_readers; t++)
-        readers.emplace_back([&] {
+        readers.emplace_back([&, t] {
             if (bind_io) bind_thread(pipe->dev);
-            if (dev_src) cudaSetDevice(pipe->dev.dev);
+            if (dev_src || staged_src) cudaSetDevice(pipe->dev.dev);
+            auto task_read = [&](Batch* b) { if (b->reads_left.fetch_sub(1) == 1) { b->t_read = now_ns(); submit_q.push(b); } };
+            PieceReader* pr = staged_src ? &pipe->readers[t] : nullptr;
+            uint8_t* const pbase = staged_src ? pipe->pieces + (size_t)t * kPieces * kPieceBytes : nullptr;
+            uint64_t piece_seq[kPieces] = {};       // sequence number of the last copy out of each piece
+            uint64_t issued = 0, done = 0;          // copies issued / known complete
+            std::deque<std::pair<Batch*, uint64_t>> pending;     // tasks read, and the copy that completes each
+            // the window being filled: slot window `win` of d_win, held in piece issued % kPieces, bytes [lo, hi) filled
+            uint8_t* d_win = nullptr; size_t win = 0, lo = 0, hi = 0;
+            auto reap = [&] {
+                while (!pending.empty() && pending.front().second <= done) { task_read(pending.front().first); pending.pop_front(); }
+            };
+            // wait until copy number `seq` has completed.  Polled: a blocking wait's wake-up left readers waiting for
+            // pieces 25-66 % of their time, polling 7-14 % (profiles/r03_piece_variants.txt)
+            auto wait_copy = [&](uint64_t seq) -> int {
+                if (seq <= done) return VMIG_OK;
+                const uint64_t w0 = now_ns();
+                cudaError_t e;
+                while ((e = cudaEventQuery(pr->ev[(seq - 1) % kPieces])) == cudaErrorNotReady) {}
+                piece_wait += now_ns() - w0;
+                if (e != cudaSuccess) { cudaGetLastError(); return fail(VMIG_ECUDA, "cudaEventQuery(piece): %s", cudaGetErrorString(e)); }
+                done = seq;
+                return VMIG_OK;
+            };
+            // every copy of this reader has completed: after an error, before idling and before exiting
+            auto drain = [&] {
+                if (!staged_src) return;
+                d_win = nullptr;
+                if (int rc = wait_copy(issued)) {
+                    set_err(rc);
+                    cudaStreamSynchronize(pr->stream); cudaGetLastError(); done = issued;
+                }
+                reap();
+            };
+            auto flush = [&]() -> int {
+                if (!d_win) return VMIG_OK;
+                const uint32_t p = (uint32_t)(issued % kPieces);
+                uint8_t* const d = d_win; d_win = nullptr;
+                CU_API(cudaMemcpyAsync(d + win * kPieceBytes + lo, pbase + (size_t)p * kPieceBytes + lo, hi - lo, cudaMemcpyHostToDevice, pr->stream));
+                CU_API(cudaEventRecord(pr->ev[p], pr->stream));
+                piece_seq[p] = ++issued;
+                return VMIG_OK;
+            };
+            auto read_part = [&](size_t i, const Piece& pc, uint8_t* d_buf) -> int {
+                if (!pc.len) return io->read_block(blocks[i], pc.off, pc.len, pbase);
+                if (d_win && (d_win != d_buf || win != pc.window)) { if (int rc = flush()) return rc; }
+                if (!d_win) {
+                    // the newest copy is usually done already: one query reaps every task it completes
+                    if (issued > done && cudaEventQuery(pr->ev[(issued - 1) % kPieces]) == cudaSuccess) { done = issued; reap(); }
+                    if (int rc = wait_copy(piece_seq[issued % kPieces])) return rc;
+                    reap();
+                    d_win = d_buf; win = pc.window; lo = kPieceBytes; hi = 0;
+                }
+                const size_t at = slot_off[i] + pc.off - win * kPieceBytes;
+                if (int rc = io->read_block(blocks[i], pc.off, pc.len, pbase + (size_t)(issued % kPieces) * kPieceBytes + at)) return rc;
+                lo = std::min(lo, at); hi = std::max(hi, at + pc.len);
+                return VMIG_OK;
+            };
             IoTask k;
-            while (read_q.pop(&k)) {
-                Slot& sl = pipe->slots[k.batch->slot];
+            for (;;) {
+                if (!read_q.try_pop(&k)) { drain(); if (!read_q.pop(&k)) break; }
+                if (err->load()) drain();
                 const uint64_t r0 = now_ns();
-                if (!err->load())
-                    for (size_t i = k.i0; i < k.i1; i++) {
-                        int rc = dev_src ? io->read_block_dev(blocks[i], sl.d_buf, slot_off[i]) : io->read_block(blocks[i], sl.h_in + slot_off[i]);
-                        if (rc) { set_err(rc); break; }
+                if (!err->load()) {
+                    uint8_t* const d_buf = pipe->slots[k.batch->slot].d_buf;
+                    int rc = VMIG_OK;
+                    for (size_t i = k.i0; i < k.i1 && !rc; i++) {
+                        if (dev_src) { rc = io->read_block_dev(blocks[i], d_buf, slot_off[i]); continue; }
+                        for (size_t j = 0, np = piece_count(slot_off[i], blocks[i].len, kPieceBytes); j < np && !rc; j++)
+                            rc = read_part(i, block_piece(slot_off[i], blocks[i].len, kPieceBytes, 0, j), d_buf);
                     }
+                    if (!rc && staged_src) rc = flush();
+                    if (rc) set_err(rc);
+                }
                 rd_busy += now_ns() - r0;
-                if (k.batch->reads_left.fetch_sub(1) == 1) { k.batch->t_read = now_ns(); submit_q.push(k.batch); }
+                if (!staged_src) { task_read(k.batch); continue; }
+                pending.emplace_back(k.batch, issued);
+                if (err->load()) drain(); else reap();
             }
+            drain();
         });
 
     // ---- stage 3: submit H2D + kernel (+ D2H) on the slot's side stream
@@ -630,8 +751,7 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
                 h2d += r.len;
             }
         } else {
-            // (GPUDirect Storage backends already put the bytes into the HBM slot on the reader threads)
-            if (!dev_src) CU_API(cudaMemcpyAsync(sl.d_buf, sl.h_in, b->bytes_used, cudaMemcpyHostToDevice, sl.stream));
+            // the reader threads already put the bytes into the HBM slot
             for (uint32_t i = 0; i < n; i++) h2d += blocks[b->b0 + i].len;
         }
         HashLaunch a;
@@ -811,14 +931,16 @@ int run_lane(Pipe* pipe, const std::vector<BlockRef>& blocks, BlockIO* io, bool 
             a[2] += (b.t_hash - b.t_sub) / 1e6; a[3] += (b.t_d2h - b.t_hash) / 1e6; a[4] += (b.t_done - b.t_d2h) / 1e6; nb++;
         }
         fprintf(stderr, "[vmig trace] gpu %d: %zu batches in %.1f ms; mean ms/batch: read %.2f submit-wait %.2f h2d+hash %.2f d2h %.2f write %.2f; "
-                        "reader busy %.0f%% of %u, writer busy %.0f%% of %u; dispatcher waited %.1f ms for slots; kernel sum %.1f ms\n",
+                        "reader busy %.0f%% of %u, writer busy %.0f%% of %u; dispatcher waited %.1f ms for slots; kernel sum %.1f ms; "
+                        "readers waited %.1f ms for pieces\n",
                 pipe->dev.dev, nb, wall, a[0] / nb, a[1] / nb, a[2] / nb, a[3] / nb, a[4] / nb,
                 100.0 * rd_busy.load() / 1e6 / (wall * n_readers), n_readers, 100.0 * wr_busy.load() / 1e6 / (wall * n_writers), n_writers,
-                slot_wait.load() / 1e6, stats->ms_kernel);
+                slot_wait.load() / 1e6, stats->ms_kernel, piece_wait.load() / 1e6);
     }
     // the slots go back to the pool idle
     cudaSetDevice(pipe->dev.dev);
     for (auto& s : pipe->slots) cudaStreamSynchronize(s.stream);
+    for (auto& r : pipe->readers) cudaStreamSynchronize(r.stream);
     return err->load();
 }
 

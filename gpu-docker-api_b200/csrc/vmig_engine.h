@@ -1,13 +1,13 @@
 // vmig_engine.h -- per-GPU streaming pipeline of libvmig (internal interface).
 //
-//   source blocks --(reader threads: pread / memcpy)--> pinned IN slot
-//       --cudaMemcpyAsync H2D (slot's side stream)--> HBM slot
+//   source blocks --(reader threads: pread / memcpy, 1 MiB at a time)--> the reader's own pinned pieces
+//       --cudaMemcpyAsync H2D per piece (the reader's stream)--> HBM slot
 //       --xxh64_blocks kernel (+ compare with prior table)--> hashes, changed flags
 //       --cudaMemcpyAsync D2H of the surviving blocks--> pinned OUT slot
 //       --(writer threads: pwrite / memcpy)--> destination
 //
-// One Pipe owns kSlots such slot triples on one GPU; a lane (one GPU's share of one call) checks
-// a Pipe out of the process-wide pool, runs its block list through it and returns it.
+// One Pipe owns VMIG_SLOTS slots (HBM buffer + pinned OUT buffer) and the readers' pieces on one GPU; a lane (one GPU's
+// share of one call) checks a Pipe out of the process-wide pool, runs its block list through it and returns it.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -45,7 +45,9 @@ struct BlockRef {
 class BlockIO {
 public:
     virtual ~BlockIO() {}
-    virtual int  read_block(const BlockRef& b, uint8_t* dst) = 0;
+    // bytes [off, off + len) of block b into dst; off and len come from block_piece() (vmig_common.h), and dst has room
+    // for the piece's io_len
+    virtual int  read_block(const BlockRef& b, size_t off, size_t len, uint8_t* dst) = 0;
     virtual int  write_block(const BlockRef& b, const uint8_t* src) = 0;
     // called exactly once per block when it needs nothing more (written == false: skipped)
     virtual int  block_done(const BlockRef&, bool /*written*/) { return VMIG_OK; }

@@ -90,14 +90,15 @@ const char* vmig_version(void);
 
 #define VMIG_F_DIRECT_IO         0x80u  /* disk-backed trees (the documented deployment keeps the Docker root on
                                            xfs/LVM: reference docs/volume/volume-size-scale-en.md:5-21): source
-                                           files are read with O_DIRECT straight INTO the pinned staging ring and
-                                           destination files written with O_DIRECT straight OUT of it -- the NVMe
-                                           DMAs to/from the same page-locked memory the GPU's copy engines use, and
+                                           files are read with O_DIRECT straight INTO the readers' pinned pieces
+                                           and destination files written with O_DIRECT straight OUT of the pinned
+                                           OUT ring -- the NVMe DMAs to/from the same page-locked memory the
+                                           GPU's copy engines use, and
                                            the page cache (two CPU copies per byte) is bypassed.  Falls back to
                                            buffered I/O per file where the filesystem refuses O_DIRECT.  Env
                                            VMIG_DIRECT_IO=1 sets it for every call.                              */
 #define VMIG_F_CUFILE            0x100u /* GPUDirect Storage: source blocks are read with cuFileRead straight into the
-                                           HBM slot (no IN ring, no H2D copy) and surviving blocks written with
+                                           HBM slot (no pinned pieces, no H2D copy) and surviving blocks written with
                                            cuFileWrite straight out of it (no D2H copy, no OUT ring).  libcufile is
                                            dlopen()ed: VMIG_EINVAL if it cannot be loaded or its driver cannot be
                                            opened, VMIG_EIO with libcufile's own reason if it refuses a descriptor
